@@ -32,6 +32,8 @@ MIB = 1 << 20
 SEED0 = 0x5EA3EED5F00DCAFE
 METRIC = "rs10_4_encode_input_GBps"
 UNIT = "GB/s"
+DUMP_BYTES_PER_SHARD = 1 << 21      # --dump-outputs: 4 shards x 2 Mi positions as float32 = 32 MiB
+DUMP_SEED = 0x5EED
 
 
 def load_traffic(dat_size):
@@ -281,6 +283,22 @@ def oracle_window_check(par, dat_size, shard, seed, offs=None):
     return len(offs)
 
 
+def dump_outputs(out_dir, par, shard):
+    """--dump-outputs: the four parity shards the last timed step wrote, as DIR/ec10.npy … ec13.npy (float32, one
+    value per byte).  A shard longer than DUMP_BYTES_PER_SHARD is sampled at the same seeded, sorted positions on
+    every run, so two builds given the same arguments can be compared output for output."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    if shard > DUMP_BYTES_PER_SHARD:
+        pos = np.sort(np.random.default_rng(DUMP_SEED).choice(shard, DUMP_BYTES_PER_SHARD, replace=False))
+    else:
+        pos = np.arange(shard)
+    idx = torch.from_numpy(pos).to(par[0].device)
+    for p in range(4):
+        np.save(os.path.join(out_dir, "ec%02d.npy" % (10 + p)), par[p][idx].float().cpu().numpy())
+
+
 def whole_volume_check(L, local, par_ptrs, par, dat_size, shard, seed, stream):
     """Every byte of the four parity shards of one encoded volume against the CPU oracle: the device digests of the
     shards must equal the digests oracle/cpu_baseline.c::orc_volume_digests computes for the same seeded volume
@@ -504,6 +522,9 @@ def main():
     ap.add_argument("--no-host-api", action="store_true", help="skip the Encoder-level host-buffer leg")
     ap.add_argument("--batch-leg-volumes", type=int, default=256,
                     help="volumes of the configs[3] batch leg inside the default line (0 = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write rank 0's parity shards of the last step to DIR/ec10.npy … "
+                         "ec13.npy (float32, a fixed seeded sample of byte positions)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "swec" else args.warmup
     if args.impl == "reference":
@@ -658,6 +679,8 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms_max = float(t.item())
     value = world * args.steps * dat_size / (ms_max / 1e3) / 1e9
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, par, shard)
 
     # correctness outside the timed region: spot-check the parity against the oracle (rank 0)
     checked = None

@@ -10,7 +10,8 @@ import pytest
 pytestmark = pytest.mark.gpu
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_DAT = os.path.join(ROOT, "oracle", "_ref", "1.dat")
+FIXTURES = os.path.join(ROOT, "tests", "golden", "fixtures")
+FIXTURE_DAT = os.path.join(FIXTURES, "1.dat")
 SEED = 0x5EA3EED5F00DCAFE
 
 
@@ -407,9 +408,7 @@ def test_encode_volume_device_layout(cuda, enc, oracle, size, large, small):
 
 def test_fixture_1dat_digests(cuda, enc, kat):
     """K8: the reference's own fixture volume, shards byte-identical to the reference arithmetic."""
-    if not os.path.exists(REF_DAT):
-        pytest.skip("oracle/_ref/1.dat not shipped")
-    dat = np.fromfile(REF_DAT, dtype=np.uint8)
+    dat = np.fromfile(FIXTURE_DAT, dtype=np.uint8)
     for label in ("production", "test"):
         g = kat["K8"][label]
         got = encode_volume_on_device(cuda, enc, dat, g["large"], g["small"])
@@ -487,29 +486,28 @@ def test_verify_ec_files_scrub(cuda, swec, oracle, tmp_path):
 
 
 def test_generate_ec_files_test_parameters_and_fixture(cuda, swec, oracle, kat, tmp_path):
-    """TestEncodingDecoding (ec_test.go:23-47): generateEcFiles("1", 50, 10000, 100) on the fixture volume."""
+    """TestEncodingDecoding (ec_test.go:23-47): generateEcFiles("1", 50, 10000, 100) on the fixture volume (its shards
+    also carry the reference kernel's digests, K8) and on a synthetic volume the size of the reference's 1.dat."""
     ec = swec.erasure_coding
-    if os.path.exists(REF_DAT):
-        dat = np.fromfile(REF_DAT, dtype=np.uint8)
-    else:
-        dat = oracle.synth(0, 2_590_912, SEED)
-    base = str(tmp_path / "1")
-    dat.tofile(base + ".dat")
-    ec.generateEcFiles(base, 50, 10000, 100)
-    want = oracle.encode_dat_image(dat, buffer_size=50, large=10000, small=100)
-    for i in range(14):
-        assert (np.fromfile(base + ec.ToExt(i), dtype=np.uint8) == want[i]).all(), i
-    if os.path.exists(REF_DAT):
-        digests = [hashlib.sha256(open(base + ec.ToExt(i), "rb").read()).hexdigest() for i in range(14)]
-        assert digests == kat["K8"]["test"]["sha256"]
-    # rebuild with a .vif that carries the ratio (ec_encoder.go:76-95); reference quirk: shards above
-    # 1 MiB must be 1 MiB multiples, these are 259,100 B (< 1 MiB) so one short read is fine
-    open(base + ".vif", "w").write('{\n  "version": 3,\n  "datFileSize": "%d",\n  "ecShardConfig": {\n    "dataShards": 10,\n    "parityShards": 4\n  }\n}\n' % len(dat))
-    os.remove(base + ".ec02")
-    os.remove(base + ".ec12")
-    assert ec.RebuildEcFiles(base) == [2, 12]
-    for i in (2, 12):
-        assert (np.fromfile(base + ec.ToExt(i), dtype=np.uint8) == want[i]).all()
+    for name, dat in (("fixture", np.fromfile(FIXTURE_DAT, dtype=np.uint8)), ("synthetic", oracle.synth(0, 2_590_912, SEED))):
+        (tmp_path / name).mkdir()
+        base = str(tmp_path / name / "1")
+        dat.tofile(base + ".dat")
+        ec.generateEcFiles(base, 50, 10000, 100)
+        want = oracle.encode_dat_image(dat, buffer_size=50, large=10000, small=100)
+        for i in range(14):
+            assert (np.fromfile(base + ec.ToExt(i), dtype=np.uint8) == want[i]).all(), (name, i)
+        if name == "fixture":
+            digests = [hashlib.sha256(open(base + ec.ToExt(i), "rb").read()).hexdigest() for i in range(14)]
+            assert digests == kat["K8"]["test"]["sha256"]
+        # rebuild with a .vif that carries the ratio (ec_encoder.go:76-95); reference quirk: shards above
+        # 1 MiB must be 1 MiB multiples, these are < 1 MiB so one short read is fine
+        open(base + ".vif", "w").write('{\n  "version": 3,\n  "datFileSize": "%d",\n  "ecShardConfig": {\n    "dataShards": 10,\n    "parityShards": 4\n  }\n}\n' % len(dat))
+        os.remove(base + ".ec02")
+        os.remove(base + ".ec12")
+        assert ec.RebuildEcFiles(base) == [2, 12]
+        for i in (2, 12):
+            assert (np.fromfile(base + ec.ToExt(i), dtype=np.uint8) == want[i]).all(), (name, i)
 
 
 def test_custom_ratio_from_vif(cuda, swec, oracle, tmp_path):
@@ -670,15 +668,12 @@ def test_encoding_decoding_like_ec_test_go(cuda, swec, oracle, tmp_path):
     .ec00-.ec09 equal the .dat bytes (validateFiles/assertSame) AND the same interval recovered from ten
     OTHER shards with ReconstructData equals them too (readFromOtherEcFiles — dead code in the reference)."""
     from oracle import rs_numpy as rn
-    ref_idx = os.path.join(ROOT, "oracle", "_ref", "1.idx")
-    if not (os.path.exists(REF_DAT) and os.path.exists(ref_idx)):
-        pytest.skip("oracle/_ref fixtures not shipped")
     ec = swec.erasure_coding
     large, small = 10000, 100
     base = str(tmp_path / "1")
-    dat = np.fromfile(REF_DAT, dtype=np.uint8)
+    dat = np.fromfile(FIXTURE_DAT, dtype=np.uint8)
     dat.tofile(base + ".dat")
-    open(base + ".idx", "wb").write(open(ref_idx, "rb").read())
+    open(base + ".idx", "wb").write(open(os.path.join(FIXTURES, "1.idx"), "rb").read())
     ec.WriteSortedFileFromIdx(base, ".ecx")                  # before the shards, like VolumeEcShardsGenerate
     ec.generateEcFiles(base, 50, large, small)
     shards = [np.fromfile(base + ec.ToExt(i), dtype=np.uint8) for i in range(14)]

@@ -1,6 +1,6 @@
 """Index files either side of the RS path (.idx → .ecx, .ecj fold, .ecx → .idx, FindDatFileSize):
-host-only twins in libswec against the oracle's restatement, on the reference's own fixture index
-(1.idx, 298 entries) when oracle/_ref ships it, and on synthetic indexes with overwrites/deletions."""
+host-only twins in libswec against the oracle's restatement, on the reference's fixture index
+(tests/golden/fixtures/1.idx, 110 of its entries) and on synthetic indexes with overwrites/deletions."""
 import os
 
 import numpy as np
@@ -8,9 +8,9 @@ import pytest
 
 from oracle import rs_numpy as rn
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_IDX = os.path.join(ROOT, "oracle", "_ref", "1.idx")
-REF_DAT = os.path.join(ROOT, "oracle", "_ref", "1.dat")
+FIXTURES = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "fixtures")
+FIXTURE_IDX = os.path.join(FIXTURES, "1.idx")
+FIXTURE_DAT = os.path.join(FIXTURES, "1.dat")
 
 
 def synthetic_idx(seed=4, n=500):
@@ -35,9 +35,7 @@ def synthetic_idx(seed=4, n=500):
 def test_ecx_from_idx_and_journal_fold(swec, tmp_path, source):
     ec = swec.erasure_coding
     if source == "fixture":
-        if not os.path.exists(REF_IDX):
-            pytest.skip("oracle/_ref/1.idx not shipped")
-        idx = open(REF_IDX, "rb").read()
+        idx = open(FIXTURE_IDX, "rb").read()
     else:
         idx = synthetic_idx()
     base = str(tmp_path / "1")
@@ -72,12 +70,10 @@ def test_ecx_from_idx_and_journal_fold(swec, tmp_path, source):
 def test_find_dat_file_size_on_fixture_volume(swec, oracle, tmp_path):
     """FindDatFileSize reads the needle version from the superblock at the start of .ec00 and returns the
     end of the last live needle — for the reference's fixture volume that is the .dat size itself."""
-    if not (os.path.exists(REF_IDX) and os.path.exists(REF_DAT)):
-        pytest.skip("oracle/_ref fixtures not shipped")
     ec = swec.erasure_coding
-    dat = np.fromfile(REF_DAT, dtype=np.uint8)
+    dat = np.fromfile(FIXTURE_DAT, dtype=np.uint8)
     base = str(tmp_path / "1")
-    open(base + ".idx", "wb").write(open(REF_IDX, "rb").read())
+    open(base + ".idx", "wb").write(open(FIXTURE_IDX, "rb").read())
     ec.WriteSortedFileFromIdx(base, ".ecx")
     shards = oracle.encode_dat_image(dat, buffer_size=50, large=10000, small=100)
     shards[0].tofile(base + ".ec00")

@@ -8,7 +8,7 @@ import pytest
 
 from oracle import rs_numpy as rn
 
-REF_DAT = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref", "1.dat")
+FIXTURE_DAT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "fixtures", "1.dat")
 
 
 def test_k1_log_table(kat, oracle):
@@ -65,18 +65,20 @@ def test_generator_matrix(kat, oracle):
     assert [int(p[0]) for p in oracle.encode(10, 4, data)] == [10, 11, 12, 13]
 
 
-def test_k6_reference_c_kernel_agrees(oracle):
-    if not oracle.ref_available():
-        pytest.skip("oracle/_ref not built (needs /root/reference)")
-    rng = np.random.default_rng(7)
+def test_k6_reference_c_kernel_agrees(kat, oracle):
+    """The parity the reference's compiled C kernel gave for seeded inputs (kat.json K6): the restatement, the GFNI
+    port and, where oracle/_ref is built, the reference kernel itself all reproduce it."""
     g = oracle.build_matrix(10, 14)
-    for n in (1, 15, 64, 10_003, 300_000):
-        ins = [rng.integers(0, 256, n, dtype=np.uint8) for _ in range(10)]
-        want = oracle.encode(10, 4, ins)
-        for kind in ([0, 1] if oracle.gfni_level() else [0]):
-            outs = [np.zeros(n, dtype=np.uint8) for _ in range(4)]
-            oracle.cpu_apply(kind, g[10:], ins, outs, threads=3, batch=4096)
-            assert all((a == b).all() for a, b in zip(outs, want)), (kind, n)
+    seed = int(kat["K6"]["seed"], 16)
+    for n, want in kat["K6"]["parity_sha256"].items():
+        n = int(n)
+        ins = [oracle.synth(i * n, n, seed) for i in range(10)]
+        got = {"oracle": oracle.encode(10, 4, ins)}
+        for kind in ([1] if oracle.gfni_level() else []) + ([0] if oracle.ref_available() else []):
+            got[kind] = [np.zeros(n, dtype=np.uint8) for _ in range(4)]
+            oracle.cpu_apply(kind, g[10:], ins, got[kind], threads=3, batch=4096)
+        for name, par in got.items():
+            assert [hashlib.sha256(p.tobytes()).hexdigest() for p in par] == want, (name, n)
 
 
 def test_k7_locate_data(kat, oracle):
@@ -97,16 +99,14 @@ def test_locate_data_boundary_sweep(oracle):
 
 
 def test_k8_fixture_digests(kat, oracle):
-    if not os.path.exists(REF_DAT):
-        pytest.skip("oracle/_ref/1.dat absent")
-    dat = np.fromfile(REF_DAT, dtype=np.uint8)
+    dat = np.fromfile(FIXTURE_DAT, dtype=np.uint8)
     assert hashlib.sha256(dat.tobytes()).hexdigest() == kat["K8"]["dat_sha256"]
     for label, bufsz in (("production", 256 * 1024), ("test", 50)):
         g = kat["K8"][label]
         shards = oracle.encode_dat_image(dat, buffer_size=bufsz, large=g["large"], small=g["small"])
         assert [hashlib.sha256(s.tobytes()).hexdigest() for s in shards] == g["sha256"]
         # ec_test.go:49-101 validateFiles: every byte is where LocateData says it is
-        for off, size in ((0, 1), (8, 5000), (len(dat) - 1000, 1000), (123456, 234567)):
+        for off, size in ((0, 1), (8, 5000), (len(dat) - 1000, 1000), (99000, 5000)):
             got = b""
             for iv in oracle.locate_data(g["large"], g["small"], len(dat) // 10, off, size):
                 sid, soff = rn.interval_to_shard(iv, g["large"], g["small"])

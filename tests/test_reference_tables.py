@@ -155,7 +155,7 @@ def test_ec_volume_file_and_delete_count_after_delete(swec, tmp_path):
 
 # ---- TestCheckIndexFile (weed/storage/idx/check_test.go:11-108): the reference's six index fixtures with the counts
 # ---- and the exact findings its test expects — K11 of oracle/README.md.  EcVolume.ScrubIndex runs this on .ecx.
-IDX_FIXTURES = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref", "idx_test_files")
+IDX_FIXTURES = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "fixtures", "idx")
 CHECK_INDEX_CASES = [
     ("simple_index.idx", 161, []),
     ("deleted_files.idx", 230, []),
@@ -179,8 +179,6 @@ CHECK_INDEX_CASES = [
 @pytest.mark.parametrize("name,want_count,want_errs", CHECK_INDEX_CASES, ids=[c[0] for c in CHECK_INDEX_CASES])
 def test_check_index_file_on_reference_fixtures(swec, name, want_count, want_errs):
     path = os.path.join(IDX_FIXTURES, name)
-    if not os.path.exists(path):
-        pytest.skip("oracle/_ref/idx_test_files not shipped")
     count, errs = swec.erasure_coding.CheckIndexFile(path, 3)
     assert count == want_count
     assert errs == want_errs

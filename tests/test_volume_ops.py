@@ -12,8 +12,9 @@ import pytest
 from oracle import rs_numpy as rn
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_IDX = os.path.join(ROOT, "oracle", "_ref", "1.idx")
-REF_DAT = os.path.join(ROOT, "oracle", "_ref", "1.dat")
+FIXTURES = os.path.join(ROOT, "tests", "golden", "fixtures")
+FIXTURE_IDX = os.path.join(FIXTURES, "1.idx")
+FIXTURE_DAT = os.path.join(FIXTURES, "1.dat")
 MIB = 1 << 20
 
 
@@ -225,12 +226,11 @@ def test_mounted_ec_volume_sees_journal_growth(swec, oracle, tmp_path):
 
 
 def test_ecx_search_on_reference_fixture_389(swec, tmp_path):
-    """TestPositioning (ec_volume_test.go:14-58): SearchNeedleFromSortedIndex on the reference's 389.ecx (485,098
-    entries) finds the needles of its table at the listed offsets and sizes.  The fixture has no shard files, so
-    the reads themselves stop at "too few shards" — offset and size are reported all the same."""
-    fixture = os.path.join(ROOT, "oracle", "_ref", "389.ecx")
-    if not os.path.exists(fixture):
-        pytest.skip("oracle/_ref/389.ecx not shipped")
+    """TestPositioning (ec_volume_test.go:14-58): SearchNeedleFromSortedIndex on a 2048-entry sample of the
+    reference's 389.ecx (485,098 entries) finds the needles of its table at the listed offsets and sizes.  The
+    fixture has no shard files, so the reads themselves stop at "too few shards" — offset and size are reported
+    all the same."""
+    fixture = os.path.join(FIXTURES, "389_sample.ecx")
     ec = swec.erasure_coding
     base = str(tmp_path / "389")
     os.symlink(fixture, base + ".ecx")
@@ -334,9 +334,7 @@ def test_volume_encode_rebuild_decode_cycle(cuda, swec, oracle, kat, tmp_path, v
     import hashlib
     ec = swec.erasure_coding
     if volume == "fixture":
-        if not (os.path.exists(REF_DAT) and os.path.exists(REF_IDX)):
-            pytest.skip("oracle/_ref fixtures not shipped")
-        dat, idx = np.fromfile(REF_DAT, dtype=np.uint8), open(REF_IDX, "rb").read()
+        dat, idx = np.fromfile(FIXTURE_DAT, dtype=np.uint8), open(FIXTURE_IDX, "rb").read()
     else:
         dat, idx = synthetic_volume(seed=21, needles=400)          # ≈8 MiB: one ragged small row
     base = str(tmp_path / "1")
